@@ -8,6 +8,11 @@ tensorflow-benchmarks.yaml: --model=resnet101 --batch_size=64
   python bench.py --gpus 1 --steps 20 --warmup 5
   python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
       --master-port 29511 bench.py --gpus 8 --steps 20 --warmup 5
+  python bench.py --gpus 1 --steps 20 --warmup 5 --dump-outputs /tmp/bench-outputs
+
+--dump-outputs DIR  after the timed steps, rank 0 writes what the last step left to the caller as DIR/<name>.npy
+                  (see dump_outputs); the inputs are seeded, so two builds run with the same arguments can be
+                  compared output for output
 
 --impl ours       (default) b200mpi: symmetric-window gradients, fused
                   allreduce+SGD sm_100a kernels, whole step in a CUDA graph
@@ -98,6 +103,29 @@ class ClockSampler:
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_SAMPLE = 1 << 22   # parameter elements written by --dump-outputs (16 MiB in fp32; ResNet-101 has 44.5 M)
+
+
+def dump_outputs(directory: str, loss, params, buffers) -> None:
+    """What one training step hands back to its caller, as float32 .npy files: the step's loss (``loss.npy``), the
+    fp32 master parameters after the step (``params.npy``: every parameter flattened in NCHW order and concatenated in
+    ``module.parameters()`` order; above DUMP_SAMPLE elements the ones at DUMP_SAMPLE distinct positions drawn by
+    ``numpy.random.default_rng(0)``, in ascending order) and the module's floating-point buffers (``buffers.npy``:
+    BatchNorm running statistics, concatenated in ``module.buffers()`` order)."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    flat = torch.cat([p.detach().float().reshape(-1) for p in params])
+    n = flat.numel()
+    if n > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(n, size=DUMP_SAMPLE, replace=False))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    np.save(os.path.join(directory, "params.npy"), flat.cpu().numpy())
+    np.save(os.path.join(directory, "loss.npy"), loss.detach().float().cpu().numpy())
+    bufs = [b.detach().float().reshape(-1) for b in buffers if b.is_floating_point()]
+    np.save(os.path.join(directory, "buffers.npy"), torch.cat(bufs).cpu().numpy() if bufs else np.zeros(0, np.float32))
+
+
 def _clean_child_env(port_shift: int, job_suffix: str, extra: dict) -> dict:
     """Environment of a child measurement: its own rendezvous port and job id, and NOT torchrun's agent-store settings -
     with TORCHELASTIC_USE_AGENT_STORE=True every rank (rank 0 included) only CONNECTS to MASTER_PORT expecting the agent's
@@ -111,7 +139,7 @@ def _clean_child_env(port_shift: int, job_suffix: str, extra: dict) -> dict:
     return env
 
 
-def _run_child(args, impl: str, env: dict, timeout: int):
+def _run_child(args, impl: str, env: dict, timeout: int, dump_dir: str | None = None):
     """One measurement in a child process (this rank's GPU). Returns (rc, parsed JSON line or None, stderr tail)."""
     cmd = [sys.executable, os.path.abspath(__file__), "--impl", impl, "--child", "--gpus", str(args.gpus), "--steps", str(args.steps),
            "--warmup", str(args.warmup), "--model", args.model, "--batch-size", str(args.batch_size), "--dtype", args.dtype,
@@ -124,6 +152,8 @@ def _run_child(args, impl: str, env: dict, timeout: int):
         cmd += ["--algo", args.algo]
     if args.bucket_mb:
         cmd += ["--bucket-mb", str(args.bucket_mb)]
+    if dump_dir:
+        cmd += ["--dump-outputs", dump_dir]
     try:
         p = subprocess.Popen(cmd, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, start_new_session=True)
         try:
@@ -210,7 +240,9 @@ def supervise(args) -> int:
                 if not room:
                     notes.append(f"{name}: not tried (time budget)")
                     continue
-            rc, d, err = _run_child(args, "ours", _clean_child_env(17 * k, f"ours-{name}", extra), args.attempt_timeout)
+            # every candidate dumps into the scratch directory; only the one that is reported is moved to --dump-outputs
+            cand_dump = os.path.join(workdir, f"dump-{name}") if args.dump_outputs else None
+            rc, d, err = _run_child(args, "ours", _clean_child_env(17 * k, f"ours-{name}", extra), args.attempt_timeout, cand_dump)
             ok_local = (rc == 0) and (rank != 0 or (d is not None and d.get("value")))
             ok = _agree(workdir, f"attempt{k}", rank, world, ok_local, args.attempt_timeout + 60) if world > 1 else ok_local
             if ok:
@@ -227,6 +259,12 @@ def supervise(args) -> int:
             print(json.dumps({"metric": "resnet101_images_per_sec", "value": None, "n_gpus": world, "impl": "ours",
                               "error": "every configuration failed", "attempts": notes}), flush=True)
         return 1
+    if rank == 0 and args.dump_outputs:
+        import shutil
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        src = os.path.join(workdir, f"dump-{used}")
+        for f in sorted(os.listdir(src)):
+            shutil.move(os.path.join(src, f), os.path.join(args.dump_outputs, f))
     if rank == 0:   # breadcrumb on stderr (the ONE stdout line comes after the baselines): survives a cut-off run in the driver's log tail
         print(f"[bench supervisor] main measurement ({used}): {json.dumps({k_: result.get(k_) for k_ in ('value', 'ms_per_step', 'n_gpus')})}; "
               f"candidates {json.dumps(tried)}; {time.time() - t_start:.0f} s so far", file=sys.stderr, flush=True)
@@ -304,8 +342,12 @@ def main() -> int:
     ap.add_argument("--attempt-timeout", type=int, default=200, help="limit for one configuration of the main measurement")
     ap.add_argument("--budget", type=int, default=int(os.environ.get("B200MPI_BENCH_BUDGET_S", 780)),
                     help="seconds the whole invocation may take; the same-box arms are skipped or shortened to stay inside it")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's loss, parameters and buffers as DIR/<name>.npy")
     ap.add_argument("--child", action="store_true", help="(internal) run the measurement in this process")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return reference_arm(args)
     if args.warmup < 3:
@@ -338,6 +380,9 @@ def main() -> int:
                               "n_gpus": int(os.environ.get("WORLD_SIZE", "1")), "config": {"selftest": True,
                               "port": os.environ.get("MASTER_PORT"), "job": os.environ.get("B200MPI_JOB_ID"),
                               "agent_store": os.environ.get("TORCHELASTIC_USE_AGENT_STORE")}, "e2e": {"value": v * 0.99}}), flush=True)
+            if args.dump_outputs:
+                import torch
+                dump_outputs(args.dump_outputs, torch.tensor(v), [torch.full((3,), v)], [])
         return 0
 
     if os.environ.get("B200MPI_FAULTHANDLER"):
@@ -486,6 +531,11 @@ def main() -> int:
     if problems:
         print(f"[bench rank {rank}] self-check FAILED: {'; '.join(problems)}", file=sys.stderr, flush=True)
         return 7
+    if args.dump_outputs and rank == 0:   # parameters are bit-identical on all ranks (checked above)
+        if args.impl == "torchddp":
+            dump_outputs(args.dump_outputs, loss, list(model.parameters()), list(model.buffers()))
+        else:
+            dump_outputs(args.dump_outputs, loss, list(trainer.state.master_state().values()), list(trainer.model.buffers()))
 
     import struct
     got = comm.host_allgather(struct.pack("dd", ms_dev, ms_e2e)) if world > 1 else [struct.pack("dd", ms_dev, ms_e2e)]

@@ -1,6 +1,8 @@
 """API defaulting + validation, ported as *specs* from the reference tables
 (pkg/apis/kubeflow/v2beta1/default_test.go:24-164,
 pkg/apis/kubeflow/validation/validation_test.go:29-415)."""
+import os
+
 import pytest
 
 from mpi_operator_b200.api import constants as C
@@ -9,6 +11,7 @@ from mpi_operator_b200.api.defaults import set_defaults_mpijob
 from mpi_operator_b200.api.types import MPIJob, MPIJobSpec, ReplicaSpec, RunPolicy, SchedulingPolicy
 from mpi_operator_b200.api.validation import (ERR_INVALID, ERR_NOT_SUPPORTED, ERR_REQUIRED, validate_mpijob)
 
+REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ONE_CONTAINER = {"spec": {"containers": [{}]}}
 
 
@@ -55,7 +58,7 @@ def test_defaults_replica_overrides_kept():
 
 
 def test_defaults_idempotent_and_roundtrip():
-    j = yaml_io.load_file("/root/repo/examples/pi/pi.yaml")[0]
+    j = yaml_io.load_file(os.path.join(REPO, "examples", "pi", "pi.yaml"))[0]
     a = set_defaults_mpijob(j.deepcopy())
     assert set_defaults_mpijob(a.deepcopy()) == a
     assert MPIJob.from_dict(a.to_dict()) == a
@@ -131,9 +134,10 @@ def test_aggregate_format():
 
 
 def test_reference_examples_load_and_validate():
+    """The upstream project's v2beta1 example manifests, stored unmodified under tests/golden/reference_examples."""
     for f in ["pi/pi.yaml", "pi/pi-intel.yaml", "pi/pi-mpich.yaml", "horovod/tensorflow-mnist.yaml",
               "tensorflow-benchmarks/tensorflow-benchmarks.yaml"]:
-        jobs = yaml_io.load_file("/root/reference/examples/v2beta1/" + f)
+        jobs = yaml_io.load_file(os.path.join(REPO, "tests", "golden", "reference_examples", f))
         assert len(jobs) == 1 and not validate_mpijob(set_defaults_mpijob(jobs[0]))
 
 

@@ -1,5 +1,6 @@
 """Object store / clientset / fake / informers / listers / apply configurations / workqueue
 (reference machinery: pkg/client/**, client-go workqueue)."""
+import os
 import threading
 import time
 
@@ -11,6 +12,8 @@ from mpi_operator_b200.client import (ApiError, Clientset, FakeClientset, Object
 from mpi_operator_b200.client import applyconfiguration as ac
 from mpi_operator_b200.controller.workqueue import (BucketRateLimiter, ItemExponentialFailureRateLimiter, MaxOfRateLimiter,
                                                     RateLimitingQueue)
+
+REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _pod(name, ns="default", labels=None, owner=None):
@@ -110,7 +113,7 @@ def test_store_journal_replay_compaction_and_torn_tail(tmp_path):
 
 def test_clientset_typed_roundtrip_label_selector_and_delete_collection():
     cs = Clientset(ObjectStore())
-    job = yaml_io.load_file("/root/repo/examples/pi/pi.yaml")[0]
+    job = yaml_io.load_file(os.path.join(REPO, "examples", "pi", "pi.yaml"))[0]
     c = cs.kubeflow_v2beta1().mpijobs("team-a")
     created = c.create(job)
     assert created.namespace == "team-a" and created.uid

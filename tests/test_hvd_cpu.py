@@ -92,7 +92,7 @@ def test_trace_export_and_roofline_report(tmp_path):
     ev = json.load(open(out))["traceEvents"]
     assert sum(1 for e in ev if e["ph"] == "X") == 3 and {e["pid"] for e in ev} == {0, 1}
     assert trace.summarize(trace.load_jsonl(str(p)))["allreduce[oneshot]"] == {"calls": 2, "bytes": 2048}
-    md = roofline.report("/root/repo/profiles/allreduce_sweep_n8_f32.json")
+    md = roofline.report(os.path.join(_repo(), "profiles", "allreduce_sweep_n8_f32.json"))
     assert "| float32 | 1073741824 | nvls" in md and "x |" in md
 
 

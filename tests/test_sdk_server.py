@@ -14,6 +14,8 @@ from mpi_operator_b200.cmd.options import ServerOption, parse
 from mpi_operator_b200.cmd.server import LeaderElector, Operator
 from mpi_operator_b200.client import ObjectStore
 
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
 
 def _free_port():
     s = socket.socket()
@@ -203,22 +205,11 @@ def test_auth_token_file_protects_the_object_api(tmp_path, monkeypatch):
 
 
 def test_models_match_the_reference_sdk_when_installed():
-    """Parity against the UNMODIFIED reference SDK installed at baseline/_ref (pip --target of
-    /root/reference/sdk/python/v2beta1): same openapi_types and attribute_map for all 9 MPIJob models."""
-    import os
-    import subprocess
-    import sys
-    ref = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-    if not os.path.isdir(os.path.join(ref, "mpijob")):
-        pytest.skip("reference SDK not installed (baseline/_ref)")
-    code = ("import sys, json; sys.path.insert(0, %r)\n"
-            "import mpijob.models as m\n"
-            "names = [n for n in dir(m) if n.startswith('V2beta1')]\n"
-            "print(json.dumps({n: [getattr(m, n).openapi_types, getattr(m, n).attribute_map] for n in names}))\n") % ref
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
-    if r.returncode != 0:
-        pytest.skip("reference SDK not importable here: " + r.stderr[-200:])
-    theirs = json.loads(r.stdout)
+    """Parity with the upstream, unmodified Python SDK (sdk/python/v2beta1): same openapi_types and attribute_map for all
+    9 MPIJob models. tests/golden/sdk_v2beta1_models.json holds {name: [openapi_types, attribute_map]} as read from
+    that package's `mpijob.models`."""
+    with open(os.path.join(GOLDEN, "sdk_v2beta1_models.json")) as f:
+        theirs = json.load(f)
     assert sorted(theirs) == sorted(n for n in mpijob.models.MODEL_CLASSES if n.startswith("V2beta1"))
     for name, (types, amap) in theirs.items():
         ours = mpijob.models.MODEL_CLASSES[name]
@@ -232,39 +223,12 @@ def test_models_match_the_reference_sdk_when_installed():
 
 def test_generic_models_match_the_reference_sdk_when_installed():
     """The 100 generic apimachinery models (sdk/meta_models.py, one schema table) against the generated files of the
-    UNMODIFIED reference SDK at baseline/_ref: same class names, module names, attribute maps and required fields."""
-    import os
-    import subprocess
-    import sys
+    upstream, unmodified Python SDK: same class names, module names, attribute maps and required fields.
+    tests/golden/sdk_generic_models.json holds {class: [attribute_map, required fields, module]} for every generated
+    model file of that package except the V2beta1 ones; a field is required when its setter rejects None."""
     from mpi_operator_b200.sdk.meta_models import snake
-    ref = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-    if not os.path.isdir(os.path.join(ref, "mpijob")):
-        pytest.skip("reference SDK not installed (baseline/_ref)")
-    code = ("import sys, json, inspect; sys.path.insert(0, %r)\n"
-            "import mpijob.models as m\n"
-            "import importlib, pkgutil\n"
-            "out = {}\n"
-            "for info in pkgutil.iter_modules(m.__path__):            # every generated FILE (the package __init__ lists only half)\n"
-            "    mod = importlib.import_module('mpijob.models.' + info.name)\n"
-            "    cs = [c for c in vars(mod).values() if inspect.isclass(c) and c.__module__ == mod.__name__ and hasattr(c, 'attribute_map')]\n"
-            "    if len(cs) != 1 or cs[0].__name__.startswith('V2beta1'):\n"
-            "        continue\n"
-            "    c, n = cs[0], cs[0].__name__\n"
-            "    req = []\n"
-            "    for a in c.openapi_types:\n"
-            "        try:\n"
-            "            o = c.__new__(c); o.local_vars_configuration = type('C', (), {'client_side_validation': True})()\n"
-            "            setattr(o, a, None)\n"
-            "        except ValueError:\n"
-            "            req.append(a)\n"
-            "        except Exception:\n"
-            "            pass\n"
-            "    out[n] = [c.attribute_map, sorted(req), c.__module__.rsplit('.', 1)[-1]]\n"
-            "print(json.dumps(out))\n") % ref
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, cwd="/tmp")
-    if r.returncode != 0:
-        pytest.skip("reference SDK not importable here: " + r.stderr[-200:])
-    theirs = json.loads(r.stdout)
+    with open(os.path.join(GOLDEN, "sdk_generic_models.json")) as f:
+        theirs = json.load(f)
     assert len(theirs) == 100
     for name, (amap, required, module) in theirs.items():
         ours = mpijob.models.MODEL_CLASSES.get(name)
@@ -274,31 +238,32 @@ def test_generic_models_match_the_reference_sdk_when_installed():
         assert sorted(ours.required) == required, name
 
 
-def test_reference_sdk_example_runs_unmodified_through_the_kubernetes_shim(tmp_path):
-    """The reference's own SDK example (sdk/python/v2beta1/tensorflow-mnist.py: kubernetes.client models, the stale
-    `mpijob.V1ReplicaSpec` import, `config.load_kube_config()`, `CustomObjectsApi().create_namespaced_custom_object`) is
-    executed as is against the single-box daemon through the in-tree `kubernetes` compatibility package."""
-    import socket
-    import subprocess
-    import sys
-    ref = "/root/reference/sdk/python/v2beta1/tensorflow-mnist.py"
-    if not os.path.exists(ref):
-        pytest.skip("reference tree not mounted")
+def test_sdk_example_flow_through_the_kubernetes_shim(tmp_path, monkeypatch):
+    """The flow of the upstream SDK's example (sdk/python/v2beta1/tensorflow-mnist.py): an MPIJob assembled from
+    kubernetes.client models and the stale `mpijob.V1ReplicaSpec` name, `config.load_kube_config()` and
+    `CustomObjectsApi().create_namespaced_custom_object`, served by the single-box daemon through the in-tree `kubernetes`
+    compatibility package."""
+    from kubernetes import client, config, watch
+    from kubernetes.client import V1Container, V1ObjectMeta, V1PodSpec, V1PodTemplateSpec, V1ResourceRequirements
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     op = Operator(ServerOption(fake_gpus=2, leader_elect=False, state_dir=str(tmp_path)))
     op.serve(f"127.0.0.1:{port}")
     op.start()
     try:
-        repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-        # run a byte-identical copy from an empty directory: next to the original lies the reference's own `mpijob` package,
-        # with which the example cannot even be imported (it no longer defines V1ReplicaSpec)
-        script = tmp_path / "tensorflow-mnist.py"
-        script.write_bytes(open(ref, "rb").read())
-        r = subprocess.run([sys.executable, str(script)], capture_output=True, text=True, timeout=60, cwd=str(tmp_path),
-                           env=dict(os.environ, PYTHONPATH=repo, MPIJOB_SERVER=f"127.0.0.1:{port}"))
-        assert r.returncode == 0, r.stdout + r.stderr
-        from kubernetes import client, config, watch
-        config.load_kube_config(host=f"127.0.0.1:{port}")
+        def replica(n, name, limits):
+            # command is a plain string, as in the example; the pods get the list form
+            c = V1Container(name=name, image="docker.io/kubeflow/mpi-horovod-mnist", command="mpirun",
+                            args=["-np", "2", "python", "/examples/tensorflow_mnist.py"],
+                            resources=V1ResourceRequirements(limits=limits))
+            return mpijob.V1ReplicaSpec(replicas=n, template=V1PodTemplateSpec(spec=V1PodSpec(containers=[c])))
+        job = mpijob.V2beta1MPIJob(kind="MPIJob", api_version="kubeflow.org/v2beta1", metadata=V1ObjectMeta(name="tensorflow-mnist"),
+                                   spec=mpijob.V2beta1MPIJobSpec(slots_per_worker=1, mpi_replica_specs={
+                                       "Launcher": replica(1, "mpi-launcher", {"cpu": "1", "memory": "2Gi"}),
+                                       "Worker": replica(2, "mpi-worker", {"cpu": "2", "memory": "4Gi"})}))
+        monkeypatch.setenv("MPIJOB_SERVER", f"127.0.0.1:{port}")
+        config.load_kube_config()
+        client.CustomObjectsApi().create_namespaced_custom_object(group="kubeflow.org", version="v2beta1", namespace="default",
+                                                                  plural="mpijobs", body=job)
         api = client.CustomObjectsApi()
         job = api.get_namespaced_custom_object("kubeflow.org", "v2beta1", "default", "mpijobs", "tensorflow-mnist")
         assert job["spec"]["mpiReplicaSpecs"]["Worker"]["replicas"] == 2 and job["spec"]["slotsPerWorker"] == 1
